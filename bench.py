@@ -8,6 +8,7 @@ replay 1M x 84x84 u8 (7.06 GB ring in HBM, a 10k-frame random block tiled), batc
 A = 4, terminals ~ Bernoulli(0.005), random.seed(1), Xavier weights (RandomState(1)).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--math fp32|tcgen05]
+                  [--dump-outputs DIR]
 
 N > 1 is launched by the driver through torch.distributed.run (one rank per GPU, NCCL).  Rank 0
 prints ONE JSON line.  `value` times the fused device path with inputs resident in HBM; `e2e`
@@ -16,6 +17,11 @@ kept in lock-step, cost delivered to the callback inside train()); `roofline` co
 %globaltimer timeline of the production graph (208 profiled steps regardless of --steps) with the
 replay-gather HBM fraction and the conv-stack tensor fraction as first-class fields;
 `predict_latency` times the agent's action selection — see DESIGN.md §6.
+
+--dump-outputs DIR writes, right after the timed steps and before anything else runs, what a caller of the fused
+path holds after its last step: the weights and RMSProp state of every layer (<layer>_W.npy, <layer>_S.npy), the
+step's cost (cost.npy) and its online / target Q-values (q_online.npy, q_target.npy), all float32 (13.5 MB at A = 4).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -37,6 +43,7 @@ METRIC = "DQN training steps/sec (batch 32, 84x84x4)"
 UNIT = "steps/s"
 BLOCK = 10_000
 NUM_ACTIONS = 4
+LAYERS = ("conv1", "conv2", "conv3", "fc1", "fc2")
 
 # algorithmic MACs per sample of each GEMM-shaped kernel (SURVEY §8d), nets = 2 for forward kernels
 MAC = {"conv1": 20 * 20 * 32 * 256, "conv2": 9 * 9 * 64 * 512, "conv3": 7 * 7 * 64 * 576, "fc1": 3136 * 512}
@@ -251,6 +258,18 @@ def graph_timeline(net, mem, L, dev, stream, reps=13, batch=16, at=12):
     return out, float(np.mean(spans)) if spans else 0.0
 
 
+def dump_outputs(out_dir, net):
+    """What the last timed step left for its caller, as float32 .npy files (see the module docstring)."""
+    os.makedirs(out_dir, exist_ok=True)
+    ws, ss = net.get_weights()
+    q_online, q_target = net.last_q()
+    arrays = {"cost": net.last_costs(1), "q_online": q_online, "q_target": q_target}
+    for name, w, st in zip(LAYERS, ws, ss):
+        arrays[name + "_W"], arrays[name + "_S"] = w, st
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float32))
+
+
 def run_b200(a, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -324,6 +343,8 @@ def run_b200(a, rank, world, local_rank):
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     cost_tail = net.last_costs(min(a.steps, 8))
     assert np.isfinite(cost_tail).all(), cost_tail
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, net)
     launches = net.launches_per_step() * a.steps
 
     # ---- roofline: the in-graph timeline of the production step (same graph, PDL and branches as `value`)
@@ -488,14 +509,18 @@ def main():
     ap.add_argument("--replay", type=int, default=1_000_000)
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (b200 only)")
     a = ap.parse_args()
     assert a.warmup >= 3, "timing rules: at least 3 warm-up steps"
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if a.impl == "reference":
-        if a.steps > 5000:
-            a.steps = 5000
+        if a.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the b200 path; --impl reference has none to write")
         return run_reference(a, rank, world)
     run_b200(a, rank, world, local_rank)
 

@@ -4,12 +4,11 @@ environment; VERDICT r1 N2).
 Two interchangeable drivers produce the same :class:`Trace`:
 
   * :func:`run_reference_loop` — the REFERENCE's own `Agent` + `Statistics` (src/agent.py, src/statistics.py,
-    converted in a temp dir by tests/ref_convert.py; build container only) driven through the schedule of
-    src/main.py:130-162;
-  * :func:`run_restated_loop` — an independent restatement of that loop written for this repository (the GPU box
-    has no /root/reference).  tests/test_agent_loop.py proves, in the build container, that both drivers produce
-    bit-identical traces on the same classes; the GPU test then runs the restatement on the PRODUCT classes
-    against the golden trace the reference loop produced on the oracle classes.
+    converted in a temp dir by tests/ref_convert.py) driven through the schedule of src/main.py:130-162; it needs a
+    checkout of the original project and produces tests/golden/agent_loop_golden.npz (make_agent_golden.py);
+  * :func:`run_restated_loop` — an independent restatement of that loop written for this repository.
+    tests/test_agent_loop.py proves that it reproduces the reference loop's golden traces on the oracle classes;
+    the GPU test then runs the restatement on the PRODUCT classes against the same golden traces.
 
 Whatever `mem`, `net`, `buf` objects are passed in (reference files, oracle classes, product classes) are used only
 through the reference's call surface (SURVEY §8b)."""

@@ -1,5 +1,6 @@
-"""Checkpoint fixtures shared by the CPU and GPU tests: the reference's snapshot weights (data) and a writer that
-rebuilds a checkpoint FILE with the reference's own pickle structure around them."""
+"""Checkpoint fixtures shared by the CPU and GPU tests: the reference's snapshot weights (data, fc1 sampled — see
+tests/golden/make_snapshot_fixture.py) and a writer that rebuilds a checkpoint FILE with the reference's own pickle
+structure around them."""
 import json
 import os
 import pickle
@@ -14,12 +15,26 @@ def fixture():
     return [g["W%d" % i] for i in range(5)], [g["S%d" % i] for i in range(5)], g["q_kat"]
 
 
+def game_fixture(name):
+    """(W, S) of the breakout fixture with fc2 replaced by snapshot `name`'s fc2 columns of the kept fc1 units."""
+    g = np.load(os.path.join(GOLDEN, "snapshot_breakout_77.npz"))
+    ws, ss, _ = fixture()
+    w4, s4 = g[name + "/W4"], g[name + "/S4"]
+    ws[4] = np.zeros((w4.shape[0], ws[4].shape[1]), np.float32)
+    ss[4] = np.zeros_like(ws[4])
+    ws[4][:, g["fc1_units"]] = w4
+    ss[4][:, g["fc1_units"]] = s4
+    return ws, ss
+
+
 def rebuild(skel, arrays):
     """Inverse of make_snapshot_fixture.skeleton(): arrays are consumed in traversal order."""
     if isinstance(skel, dict):
         if skel.get("__ndarray__"):
             a = next(arrays)
-            assert list(a.shape) == skel["shape"] or skel["shape"][0] == 18, (a.shape, skel["shape"])
+            # only fc2 (the one layer with 512 columns) may have another number of rows: the action count
+            assert list(a.shape) == skel["shape"] or (skel["shape"][1:] == [512] and a.shape[1:] == (512,)), \
+                (a.shape, skel["shape"])
             return a
         if "__seq__" in skel:
             items = [rebuild(v, arrays) for v in skel["items"]]

@@ -1,19 +1,13 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE_SRC = "/root/reference/src"
-HAVE_REFERENCE = os.path.isdir(REFERENCE_SRC)          # true in the build container only
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a real B200 (run by the driver with -m gpu)")
+    config.addinivalue_line("markers", "gpu: needs a real B200")
 
-
-needs_reference = pytest.mark.skipif(not HAVE_REFERENCE, reason="/root/reference only exists in the build container")

@@ -1,9 +1,9 @@
 """Generate tests/golden/agent_loop_golden.npz: traces of the REFERENCE's own control loop (src/agent.py +
 src/statistics.py, mechanically converted to Python 3 in a temp dir) driving the reference's unmodified
 replay_memory.py / state_buffer.py and the numpy DQN oracle through the schedule of src/main.py:130-162, on the
-deterministic synthetic environment.  Build container only:
+deterministic synthetic environment:
 
-    python tests/golden/make_agent_golden.py
+    python tests/golden/make_agent_golden.py <simple_dqn checkout>
 
 Cases: "breakout10k" = BASELINE configs[0] shape (replay 10k, batch 32, history 4, A = 4, train_repeat 1);
 "pong_repeat2" = A = 6 with --train_repeat 2 and target syncs every 120 steps (configs[2]'s periodic
@@ -45,6 +45,7 @@ def top2_gap(q_rows):
 def main():
     out = {}
     with tempfile.TemporaryDirectory() as tmp:
+        assert RC.convert(tmp) == {"agent.py": 7, "statistics.py": 6}      # the whole py2 -> py3 conversion: 13 lines
         for name, spec in CASES.items():
             cfg, tr = run_case(name, spec, tmp)
             arr = tr.arrays()
@@ -59,4 +60,7 @@ def main():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        sys.exit("usage: make_agent_golden.py <simple_dqn checkout>")
+    RC.REFERENCE_SRC = os.path.join(sys.argv[1], "src")
     main()

@@ -1,8 +1,7 @@
-"""Generate tests/golden/replay_golden.npz by running the UNMODIFIED reference files
-/root/reference/src/replay_memory.py and /root/reference/src/state_buffer.py.
+"""Generate tests/golden/replay_golden.npz and replay_live_golden.npz by running the UNMODIFIED files
+src/replay_memory.py and src/state_buffer.py of the original simple_dqn project:
 
-Run in the build container only (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <simple_dqn checkout>
 
 The only accommodation is the numpy shim of SURVEY §8(c): numpy >= 2 removed the
 ability to use the abstract ``np.integer`` as a dtype (replay_memory.py:11), so the
@@ -20,7 +19,6 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF_SRC = "/root/reference/src"
 
 from oracle.replay_oracle import indexed_episode_stream, decode_frame_tag  # noqa: E402
 
@@ -35,8 +33,8 @@ CASES = [
 ]
 
 
-def load_reference():
-    sys.path.insert(0, REF_SRC)
+def load_reference(ref_src):
+    sys.path.insert(0, ref_src)
     import replay_memory
     import state_buffer
     shim = types.SimpleNamespace(**{k: getattr(np, k) for k in dir(np) if not k.startswith("__")})
@@ -49,8 +47,27 @@ def crc(a):
     return np.uint32(zlib.crc32(np.ascontiguousarray(a).tobytes()))
 
 
-def main():
-    replay_memory, state_buffer = load_reference()
+def live_case(replay_memory):
+    """A ring of 500 wrapped by 1300 adds and 20 minibatches from random.seed(99), in the order the replay oracle
+    draws them (tests/test_oracle_replay.py::test_replay_oracle_live_against_reference_file)."""
+    args = types.SimpleNamespace(screen_height=84, screen_width=84, history_length=4, batch_size=32)
+    mem = replay_memory.ReplayMemory(500, args)
+    for (a, r, s, t) in indexed_episode_stream(1300, seed=3, terminal_p=0.03):
+        mem.add(a, r, s, t)
+    random.seed(99)
+    out = {"mt_before": np.array(random.getstate()[1], dtype=np.uint32)}
+    rows = {k: [] for k in ("pre_crc", "post_crc", "actions", "rewards", "terminals")}
+    for _ in range(20):
+        pre, a, r, post, t = mem.getMinibatch()
+        rows["pre_crc"].append(crc(pre)); rows["post_crc"].append(crc(post))
+        rows["actions"].append(a.copy()); rows["rewards"].append(r.copy()); rows["terminals"].append(t.copy())
+    out.update({k: np.stack(v) for k, v in rows.items()})
+    out["mt_after"] = np.array(random.getstate()[1], dtype=np.uint32)
+    return out
+
+
+def main(ref_src):
+    replay_memory, state_buffer = load_reference(ref_src)
     out = {}
     names = []
     for (name, size, steps, batch, tp, seed, nmb) in CASES:
@@ -94,7 +111,12 @@ def main():
     path = os.path.join(HERE, "replay_golden.npz")
     np.savez_compressed(path, **out)
     print("wrote", path, os.path.getsize(path), "bytes")
+    path = os.path.join(HERE, "replay_live_golden.npz")
+    np.savez_compressed(path, **live_case(replay_memory))
+    print("wrote", path, os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit("usage: make_golden.py <simple_dqn checkout>")
+    main(os.path.join(sys.argv[1], "src"))

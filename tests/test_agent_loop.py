@@ -2,22 +2,20 @@
 of the drop-in boundary — BASELINE configs[0] (replay 10k, batch 32, history 4) and the periodic target sync of
 configs[2], on the deterministic synthetic environment (ALE is not installed).
 
-CPU tests (here):
-  * [build container] the mechanically converted reference Agent + Statistics, driving the UNMODIFIED reference
-    replay_memory.py / state_buffer.py and the numpy DQN oracle, reproduce tests/golden/agent_loop_golden.npz;
-  * [everywhere] this repository's restatement of the loop (tests/agent_loop.py) on the oracle classes reproduces
-    the same golden traces: every action, the `random` stream position at every phase boundary, the replay
+CPU tests (here): tests/golden/agent_loop_golden.npz holds the traces of the mechanically converted reference
+Agent + Statistics driving the UNMODIFIED reference replay_memory.py / state_buffer.py and the numpy DQN oracle
+(tests/golden/make_agent_golden.py); this repository's restatement of the loop (tests/agent_loop.py) on the oracle
+classes reproduces those golden traces: every action, the `random` stream position at every phase boundary, the replay
     cursor, every cost and Q row — so the restatement IS the reference loop, and ReplayOracle / StateBufferOracle
     are the reference's replay / state buffer, as far as the loop can tell.
 GPU test: tests/test_gpu_agent_loop.py runs the restatement on the product classes."""
 import os
-import tempfile
 
 import numpy as np
 import pytest
 
 import agent_loop as AL
-from conftest import GOLDEN, needs_reference
+from conftest import GOLDEN
 from synthetic_env import SyntheticEnvironment
 
 CASES = {
@@ -49,24 +47,6 @@ def assert_same_trace(tr, ref, exact_numbers):
         assert np.abs(tr["q_rows"] - ref["q_rows"]).max() <= 1e-4 * np.abs(ref["q_rows"]).max()
     # columns: steps, nr_games, average_reward, min, max, meanq, meancost, weight_updates
     assert np.allclose(tr["phase_rows"], ref["phase_rows"], rtol=1e-4, atol=1e-7)
-
-
-@needs_reference
-@pytest.mark.parametrize("name", list(CASES))
-def test_converted_reference_loop_reproduces_golden(name):
-    import ref_convert as RC
-    spec = CASES[name]
-    cfg = AL.loop_config(**spec["cfg"])
-    with tempfile.TemporaryDirectory() as tmp:
-        changed = RC.convert(tmp)
-        assert changed == {"agent.py": 7, "statistics.py": 6}          # the whole py2 -> py3 conversion: 13 lines
-        RefReplay, RefStateBuffer = RC.load_reference_replay_and_statebuffer()
-        Agent, Statistics = RC.load_agent_and_statistics(tmp, RefStateBuffer, tag="t_" + name)
-        _, _, OracleDQN = AL.oracle_classes()
-        env = SyntheticEnvironment(spec["num_actions"], seed=spec["env_seed"])
-        tr = AL.run_reference_loop(Agent, Statistics, env, RefReplay(cfg.replay_size, cfg),
-                                   OracleDQN(env.numActions(), cfg), cfg, os.path.join(tmp, "s.csv"))
-    assert_same_trace(tr.arrays(), golden(name), exact_numbers=False)
 
 
 @pytest.mark.parametrize("name", list(CASES))

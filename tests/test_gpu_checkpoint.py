@@ -1,11 +1,12 @@
 """§8 a17 / f2: the reference's shipped checkpoints through the PRODUCT on the device.
 
-tests/golden/snapshot_breakout_77.npz holds the fp32 W and RMSProp state of /root/reference/snapshots/
-breakout_77.pkl bit for bit (generator: tests/golden/make_snapshot_fixture.py); snapshot_layouts.json holds the
-structure of both pickle layouts found in snapshots/.  The tests rebuild a checkpoint file in EACH layout around
-those weights, load it with DeepQNetwork.load_weights (src/deepqnetwork.py:188-189) and hold the device to the
-Q-value known answer of SURVEY §8(c); then train on the trained weights (every other GPU test runs on Xavier
-weights) and round-trip through save_weights (:191-192)."""
+tests/golden/snapshot_breakout_77.npz holds the fp32 W and RMSProp state of the reference's breakout_77.pkl bit for
+bit, with fc1 sampled to its 12 most active units (generator: tests/golden/make_snapshot_fixture.py), and the fc2
+columns of those units from four shipped snapshots; snapshot_layouts.json holds the structure of both pickle layouts
+found in snapshots/.  The tests rebuild a checkpoint file in EACH layout around those weights, load it with
+DeepQNetwork.load_weights (src/deepqnetwork.py:188-189) and hold the device to the fixture's Q-value known answer;
+then train on the trained weights (every other GPU test runs on Xavier weights) and round-trip through
+save_weights (:191-192)."""
 import json
 import os
 import pickle
@@ -13,17 +14,17 @@ import pickle
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, needs_reference
+from conftest import GOLDEN
 from helpers import make_args, random_minibatch, rel_l2
 from oracle import dqn_oracle as O
 
 pytestmark = pytest.mark.gpu
 MODES = ["fp32", "tcgen05"]
-KAT_Q0 = [4.052785, 3.199721, 5.557730, 4.043888]          # SURVEY §8(c), breakout_77 weights
-KAT_Q31 = [0.752620, 0.125157, 4.278520, 2.264925]
+KAT_Q0 = [4.393127, 3.402484, 5.425210, 4.558548]          # breakout_77 weights, fc1 sampled
+KAT_Q31 = [0.011635, -0.392340, 1.878573, 0.668184]
 
 
-from ckpt_helpers import fixture as _fixture, write_checkpoint as _write_checkpoint
+from ckpt_helpers import fixture as _fixture, game_fixture, write_checkpoint as _write_checkpoint
 
 
 def _net(mode, **kw):
@@ -116,16 +117,19 @@ def test_save_weights_structure_matches_reference_layout(tmp_path, layout):
         assert (l["params"]["W"] == w).all() and (l["states"][0] == s).all()
 
 
-@needs_reference
 @pytest.mark.parametrize("name,actions", [("breakout_77", 4), ("seaquest_178", 18), ("pong_141", 3),
                                           ("space_invaders_126", 6)])
-def test_live_reference_snapshots(name, actions):
-    """Build container + GPU only: the real files (both layouts, four action counts) through load_weights."""
+def test_live_reference_snapshots(tmp_path, name, actions):
+    """Each shipped snapshot's layout and action count through load_weights: the fixture's conv and fc1 layers with
+    that snapshot's fc2 columns of the fixture's fc1 units."""
     from simple_dqn_b200 import DeepQNetwork
-    path = "/root/reference/snapshots/%s.pkl" % name
+    path = str(tmp_path / ("%s.pkl" % name))
+    layout = "pre-1.0" if name in ("breakout_77", "pong_141") else "neon-1.3.0"
+    _write_checkpoint(path, layout, *game_fixture(name))
     net = DeepQNetwork(actions, make_args(), math_mode="tcgen05")
     net.load_weights(path)
     ws, ss = O.load_snapshot(path)
+    assert ws[4].shape == (actions, 512)
     states = np.random.RandomState(1234).randint(0, 256, (32, 4, 84, 84)).astype(np.uint8)
     ref = O.forward(ws, states)
     assert np.abs(net.predict(states) - ref).max() <= 1e-3 * np.abs(ref).max()

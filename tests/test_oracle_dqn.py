@@ -1,11 +1,14 @@
 """Cross-check the numpy Nature-DQN oracle against an independent torch-CPU autograd
-implementation, and (build container only) against the shipped snapshot KAT of SURVEY §8(c).
+implementation, and against the Q-value KAT of the shipped breakout_77 snapshot (tests/golden).
 The Neon arithmetic itself cannot be run anywhere (parity unpinned — see oracle/__init__.py)."""
+import json
+import os
+
 import numpy as np
-import pytest
 import torch
 
-from conftest import needs_reference
+from ckpt_helpers import fixture
+from conftest import GOLDEN
 from oracle import dqn_oracle as O
 
 
@@ -73,13 +76,15 @@ def test_train_step_semantics():
     assert all((t == w).all() for t, w in zip(net.target_weights, net.weights))
 
 
-@needs_reference
 def test_snapshot_kat_breakout_77():
-    ws, ss = O.load_snapshot("/root/reference/snapshots/breakout_77.pkl")
+    """breakout_77 with fc1 sampled (tests/golden/make_snapshot_fixture.py); the full network's KAT of SURVEY §8(c)
+    was asserted when the fixture was made."""
+    ws, ss, _ = fixture()
     assert [w.shape for w in ws] == O.layer_shapes(4) == [s.shape for s in ss]
     states = np.random.RandomState(1234).randint(0, 256, (32, 4, 84, 84)).astype(np.uint8)
     q = O.forward(ws, states)
-    assert np.allclose(q[0], [4.052785, 3.199721, 5.557730, 4.043888], atol=2e-5)
-    assert np.allclose(q[31], [0.752620, 0.125157, 4.278520, 2.264925], atol=2e-5)
-    ws2, _ = O.load_snapshot("/root/reference/snapshots/seaquest_178.pkl")       # neon-1.3.0 layout
-    assert [w.shape for w in ws2] == O.layer_shapes(18)
+    assert np.allclose(q[0], [4.393127, 3.402484, 5.425210, 4.558548], atol=2e-5)
+    assert np.allclose(q[31], [0.011635, -0.392340, 1.878573, 0.668184], atol=2e-5)
+    meta = json.load(open(os.path.join(GOLDEN, "snapshot_layouts.json")))
+    sk = meta["seaquest_178"]["skeleton"]["model"]["config"]["layers"]["items"]     # neon-1.3.0 layout
+    assert [tuple(l["params"]["W"]["shape"]) for l in sk if "params" in l] == O.layer_shapes(18)

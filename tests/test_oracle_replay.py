@@ -1,16 +1,13 @@
-"""Pin the replay oracle: against CPython's ``random``, against golden vectors produced by the
-unmodified reference (tests/golden/make_golden.py), and — in the build container — against the
-reference files themselves, live."""
+"""Pin the replay oracle: against CPython's ``random`` and against golden vectors produced by the
+unmodified reference (tests/golden/make_golden.py)."""
 import os
 import random
-import sys
-import types
 import zlib
 
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, REFERENCE_SRC, needs_reference
+from conftest import GOLDEN
 from oracle.mt19937 import MT19937, twist_segmented, twist_sequential
 from oracle.replay_oracle import (ReplayOracle, StateBufferOracle, decode_frame_tag,
                                   indexed_episode_stream)
@@ -87,25 +84,18 @@ def test_state_buffer_oracle_matches_reference_golden():
     assert not buf.getStateMinibatch().any()
 
 
-@needs_reference
 def test_replay_oracle_live_against_reference_file():
-    """Run the unmodified /root/reference/src/replay_memory.py beside the oracle (numpy shim only)."""
-    sys.path.insert(0, REFERENCE_SRC)
-    import replay_memory
-    shim = types.SimpleNamespace(**{k: getattr(np, k) for k in dir(np) if not k.startswith("__")})
-    shim.integer = np.int64
-    replay_memory.np = shim
-    args = types.SimpleNamespace(screen_height=84, screen_width=84, history_length=4, batch_size=32)
-    ref = replay_memory.ReplayMemory(500, args)
+    """The oracle's minibatches equal those the unmodified reference replay_memory.py drew from the same adds and
+    the same `random` stream (tests/golden/make_golden.py::live_case)."""
+    g = np.load(os.path.join(GOLDEN, "replay_live_golden.npz"))
     mem = ReplayOracle(500)
     for (a, r, s, t) in indexed_episode_stream(1300, seed=3, terminal_p=0.03):
-        ref.add(a, r, s, t)
         mem.add(a, r, s, t)
     random.seed(99)
+    assert list(random.getstate()[1]) == [int(x) for x in g["mt_before"]]
     rng = MT19937.from_python(random)
-    for _ in range(20):
-        rp, ra, rr, rq, rt = ref.getMinibatch()
+    for i in range(20):
         op, oa, orr, oq, ot = mem.getMinibatch(rng)
-        assert (rp == op).all() and (rq == oq).all()
-        assert (ra == oa).all() and (rr == orr).all() and (rt == ot).all()
-    assert list(random.getstate()[1]) == rng.state625()
+        assert crc(op) == g["pre_crc"][i] and crc(oq) == g["post_crc"][i], i
+        assert (oa == g["actions"][i]).all() and (orr == g["rewards"][i]).all() and (ot == g["terminals"][i]).all()
+    assert rng.state625() == [int(x) for x in g["mt_after"]]
